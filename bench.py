@@ -42,6 +42,8 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-side", action="store_true", help="skip the side measurements of cfg1/cfg3/cfg4/cfg5 (default workload only)")
     ap.add_argument("--cpu-steps", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the state they computed (x, v and, if any, the rigid bodies) as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -298,6 +300,28 @@ def position_checksum(eng):
     return int(zlib.crc32(x.tobytes())), float(x.astype(np.float64).sum())
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(eng, out_dir):
+    """What a caller of the timed path receives after its last step: particle positions and velocities (and the rigid-body
+    state of workloads that have rigid bodies), fp32.  Above DUMP_LIMIT_BYTES in all, the same seeded sample of particle rows
+    is written for every array, so that two builds run with the same arguments can be compared file for file."""
+    import numpy as np
+    from positionbaseddynamics_b200 import _capi
+    out = {"x": eng.get_attr(_capi.ATTR_X), "v": eng.get_attr(_capi.ATTR_V)}
+    n = len(out["x"])
+    per_row = sum(a[0].nbytes for a in out.values())
+    if n * per_row > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // 2 // per_row, replace=False))
+        out = {k: a[rows] for k, a in out.items()}
+    if getattr(eng, "n_rb", 0):
+        out["rigid_bodies"] = eng.get_rigid_bodies()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def l2_copy_bandwidth():
     """Measured L2-resident copy bandwidth (read + write bytes of a 2 x 24 MB working set that stays in the 126 MB L2), GB/s."""
     import torch
@@ -346,6 +370,8 @@ def run_b200(args):
     ms, launches = timed_steps(eng, mode, args.steps, max(args.warmup, 3), dist)
     clocks = sampler.stop() if rank == 0 else None
     crc, xsum = position_checksum(eng)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)
     ms_t = torch.tensor([ms], device="cuda", dtype=torch.float64)
     crc_t = torch.tensor([crc], device="cuda", dtype=torch.int64)
     if dist is not None:

@@ -166,3 +166,37 @@ def bar_on_colliders(m, tolerance=0.05, sub_steps=2, max_iter=3):
     m.add_model_collider(1, 0, restitution=0.4, friction=0.3)
     m.set_contact_params(stiffness=100.0, max_iter_v=5)
     return bodies
+
+
+CONTACT_SCENES = {
+    # name: (precision of the reference build, builder on a reference build); the reference's setup of each is recorded under
+    # contacts/<name>/ in tests/golden/reference_runs.npz
+    "cloth_all_shapes": ("f64", lambda m: cloth_on_colliders(m, 24, shapes=("box", "sphere", "torus", "cylinder", "hollow_sphere", "hollow_box"))),
+    "cloth_no_torus_f32": ("f32", lambda m: cloth_on_colliders(m, 24, shapes=("box", "sphere", "cylinder", "hollow_sphere", "hollow_box"))),
+    "cloth_box_sphere_torus": ("f64", lambda m: cloth_on_colliders(m, 24, shapes=("box", "sphere", "torus"))),
+    "bar": ("f64", bar_on_colliders),
+}
+
+
+def on_recorded_colliders(m, name):
+    """The C restatement (m = CpuPbd "oracle") set up as CONTACT_SCENES[name] sets up a reference build: the same particle model and
+    constraints, and the reference's rigid bodies and collision objects as recorded.  Returns (models, rigid) in the form of
+    CpuPbd.collision_objects(), what an adapter passes to pbd_set_colliders."""
+    import reference_golden
+    p = "contacts/%s/" % name
+    if name == "bar":
+        m.add_regular_tet_model(9, 4, 4, t=(0.0, 2.0, 0.0), R=np.eye(3), scale=(3.0, 0.6, 0.6))
+        m.add_solid_constraints(0, 2, k=1.0e5, nu=0.3)
+        m.set_params(dt=0.005, sub_steps=2, max_iter=3)
+    else:
+        m.add_regular_triangle_model(24, 24, t=(-2.5, 2.2, -2.5), R=RX90, scale=(5.0, 5.0))
+        m.add_cloth_constraints(0, 4, dist_k=1.0e5)
+        m.add_bending_constraints(0, 3, 100.0)
+        m.set_params(dt=0.005, sub_steps=1, max_iter=4)
+    for row in reference_golden.get(p + "rigid_bodies"):
+        m.add_rigid_body(0.0, row[:3], (1.0, 1.0, 1.0), row[3:7])
+    models = [(int(o), int(c), float(r), float(f)) for o, c, r, f in reference_golden.get(p + "models")]
+    rigid = list(reference_golden.get(p + "rigid"))
+    m.set_colliders(models, rigid)
+    m.set_oracle_contact_params(tolerance=0.05, stiffness=100.0, max_iter_v=5)
+    return models, rigid

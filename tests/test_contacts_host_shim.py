@@ -1,14 +1,13 @@
 """CPU-side guard of the contact kernel's arithmetic: csrc/contacts.cuh compiled for the host through a test-only shim (tests/host_shim/),
-one simulated thread per particle, in lockstep with the unmodified reference (oracle/_ref, fp64).  The GPU parity tests proper are in
-tests/test_gpu_contacts.py; this one runs without a GPU and is not a product path."""
+one simulated thread per particle, in lockstep with the fp64 C restatement of the contact path, which tests/test_oracle_vs_ref.py pins to
+the unmodified reference, set up with the reference's recorded colliders.  The GPU parity tests proper are in tests/test_gpu_contacts.py;
+this one runs without a GPU and is not a product path."""
 import ctypes as C
 import os
 import subprocess
 import numpy as np
-import pytest
 
 import scenes
-from conftest import have_ref
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -19,20 +18,17 @@ class _RC(C.Structure):  # pbdk::RigidCollider
 
 
 def test_contact_kernel_arithmetic_on_the_host(tmp_path, cpu_libs):
-    if not have_ref("f64"):
-        pytest.skip("prebuilt oracle/_ref/libpbdref_f64.so not present")
     from positionbaseddynamics_b200 import _capi
     so = str(tmp_path / "libcontacts_host.so")
     subprocess.check_call(["g++", "-O1", "-shared", "-fPIC", "-I" + os.path.join(ROOT, "tests", "host_shim"), "-I" + os.path.join(ROOT, "positionbaseddynamics_b200", "csrc"),
                            "-o", so, os.path.join(ROOT, "tests", "host_shim", "run_contacts.cpp")])
     lib = C.CDLL(so)
-    m = cpu_libs.CpuPbd("ref", "f64")
-    scenes.cloth_on_colliders(m, 24, shapes=("box", "sphere", "torus", "cylinder", "hollow_sphere", "hollow_box"))
+    m = cpu_libs.CpuPbd("oracle", "f64")
+    models, rigid = scenes.on_recorded_colliders(m, "cloth_all_shapes")
     mass, _ = m.masses(); n = len(mass); h = 0.005
     rb = m.rigid_bodies(); nrb = len(rb)
     rbX = np.zeros((nrb, 4), np.float32); rbX[:, :3] = rb[:, :3]
     rbV = np.zeros((nrb, 4), np.float32); rbW = np.zeros((nrb, 4), np.float32)
-    models, rigid = m.collision_objects()
     rcs = (_RC * len(rigid))()
     for k, d in enumerate(rigid):
         rc = rcs[k]; rc.shape = int(d[0]); rc.body = int(d[1]); rc.dim[:] = [float(v) for v in d[2:5]]; rc.thickness = float(d[5]); rc.invert = -1.0 if d[6] else 1.0
@@ -46,7 +42,7 @@ def test_contact_kernel_arithmetic_on_the_host(tmp_path, cpu_libs):
         x_old = m.get("x").copy()
         m.step(1)
         x_new, v_new = m.get("x").copy(), m.get("v").copy()
-        p, b, info, rr, pt = m.contacts()
+        p, b, info = m.oracle_contacts()
         v_pre = (x_new - x_old) / h  # velocityUpdateFirstOrder: what the contact solve starts from
         pos = np.zeros((n, 4), np.float32); pos[:, :3] = x_new; pos[:, 3] = np.where(mass != 0, 1.0 / np.where(mass != 0, mass, 1.0), 0.0)
         vel = np.zeros((n, 4), np.float32); vel[:, :3] = v_pre; vel[:, 3] = mass

@@ -1,20 +1,22 @@
 """Contact path (SURVEY.md section 8 row f-4, the data-parallel part): particles of a cloth against analytic distance fields on static
-rigid bodies + the velocity-level contact solve, against the UNMODIFIED reference (oracle/_ref: DistanceFieldCollisionDetection,
-ParticleRigidBodyContactConstraint, TimeStepController::velocityConstraintProjection compiled from /root/reference)."""
+rigid bodies + the velocity-level contact solve, against the UNMODIFIED reference's DistanceFieldCollisionDetection,
+ParticleRigidBodyContactConstraint and TimeStepController::velocityConstraintProjection.  The checker is the fp64 C restatement of the
+contact path (oracle/pbd_oracle.c), which tests/test_oracle_vs_ref.py pins to the reference's recorded runs, set up with the rigid bodies
+and collision objects the reference built for the same scene (tests/scenes.py:on_recorded_colliders)."""
 import numpy as np
 import pytest
 
 import scenes
 from parity_util import rel_position_error
-from conftest import have_ref
 
 pytestmark = pytest.mark.gpu
 TOL = 1.0e-4
 ALL_SHAPES = ("box", "sphere", "torus", "cylinder", "hollow_sphere", "hollow_box")
 
 
-def _engine_from(cpu, with_colliders=True):
-    """The call sequence of INTEGRATION.md: a model built by the reference is handed to the engine through the C ABI."""
+def _engine_from(cpu, colliders=None):
+    """The call sequence of INTEGRATION.md: a model built on the CPU side is handed to the engine through the C ABI; `colliders` =
+    (models, rigid) as CpuPbd.collision_objects() returns them."""
     from positionbaseddynamics_b200 import _capi
     types, bodies, params, _ = cpu.constraints()
     off, ids = cpu.groups()
@@ -25,8 +27,8 @@ def _engine_from(cpu, with_colliders=True):
     eng.set_rigid_bodies([0.0] * len(rb), rb[:, :3], rb[:, 3:7], [(1.0, 1.0, 1.0)] * len(rb))
     eng.add_flat(types, bodies, params)
     eng.set_groups(off, ids)
-    if with_colliders:
-        models, rigid = cpu.collision_objects()
+    if colliders is not None:
+        models, rigid = colliders
         pcs = [_capi.ParticleCollider(o, c, r, f) for (o, c, r, f) in models]
         rcs = []
         for d in rigid:
@@ -47,7 +49,7 @@ def _lockstep(step_gpu, get_gpu, cpu, steps, contacts_gpu=None):
     """Per-step parity from identical states.  A contact event (a particle crossing the tolerance shell, |dv| ~ 1 m/s) that happens one
     step earlier or later in fp32 than in fp64 changes the trajectory by orders of magnitude more than any rounding, so a free-running
     fp32 trajectory cannot be held against the fp64 one over hundreds of contact events; instead the GPU state is re-synchronised with the
-    reference's before every step and each step is compared on its own: positions to 1e-4 (relative), velocities -- which is all a
+    checker's before every step and each step is compared on its own: positions to 1e-4 (relative), velocities -- which is all a
     contact changes -- to 2e-3 m/s, the contact list exactly.  A particle whose signed distance is within 1e-5 of the threshold may
     legitimately be a contact on one side only; such grazing cases are counted (and bounded), everything else must agree."""
     grazing = 0; events = 0; worst_dv = 0.0; worst_x = 0.0; bodies = set()
@@ -56,8 +58,7 @@ def _lockstep(step_gpu, get_gpu, cpu, steps, contacts_gpu=None):
         step_gpu(x, v); cpu.step(1)
         xg, vg = get_gpu()
         xc, vc = cpu.get("x"), cpu.get("v")
-        p, b, info, rr, pt = cpu.contacts()
-        assert rr == 0 and pt == 0
+        p, b, info = cpu.oracle_contacts()
         events += len(p); bodies |= set(b.tolist())
         worst_x = max(worst_x, rel_position_error(xg, xc))
         assert rel_position_error(xg, xc) <= TOL  # positions of a step do not depend on its contacts
@@ -89,15 +90,13 @@ def _lockstep(step_gpu, get_gpu, cpu, steps, contacts_gpu=None):
 @pytest.mark.parametrize("mode", [0, 1])
 def test_contact_path_vs_reference(mode, cpu_libs):
     """Cloth dropped onto a floor box, a sphere, a torus, a cylinder, a hollow sphere and a hollow box (every analytic distance field of
-    DistanceFieldCollisionDetection; rotated bodies exercise the local frames), 150 steps in lockstep with the reference (fp64): the same
+    DistanceFieldCollisionDetection; rotated bodies exercise the local frames), 150 steps in lockstep with the fp64 checker: the same
     contact list with matching contact points and normals, positions within 1e-4 and velocities within 2e-3 m/s after every step."""
-    if not have_ref("f64"):
-        pytest.skip("prebuilt oracle/_ref/libpbdref_f64.so not present on this box")
     from positionbaseddynamics_b200 import _capi
-    cpu = cpu_libs.CpuPbd("ref", "f64")
-    scenes.cloth_on_colliders(cpu, 24, shapes=ALL_SHAPES)
+    cpu = cpu_libs.CpuPbd("oracle", "f64")
+    colliders = scenes.on_recorded_colliders(cpu, "cloth_all_shapes")
     cpu.init_groups()
-    eng = _engine_from(cpu)
+    eng = _engine_from(cpu, colliders)
     eng.set_params(dt=0.005, sub_steps=1, max_iter=4)
     eng.set_mode(mode)
     n = cpu.num_particles()
@@ -108,26 +107,23 @@ def test_contact_path_vs_reference(mode, cpu_libs):
     print("lockstep, mode %d: %d contact events on bodies %s, %d grazing, worst rel pos %.2e, worst |dv| %.2e m/s" % (mode, events, sorted(bodies), grazing, worst_x, worst_dv))
     assert events > 2000 and len(bodies) >= 5 and grazing <= 3
     # free-running for the first 40 steps (the first contacts appear around step 35): still inside the tolerance
-    cpu2 = cpu_libs.CpuPbd("ref", "f64")
-    scenes.cloth_on_colliders(cpu2, 24, shapes=ALL_SHAPES)
+    cpu2 = cpu_libs.CpuPbd("oracle", "f64")
+    colliders = scenes.on_recorded_colliders(cpu2, "cloth_all_shapes")
     cpu2.init_groups()
-    eng2 = _engine_from(cpu2)
+    eng2 = _engine_from(cpu2, colliders)
     eng2.set_params(dt=0.005, sub_steps=1, max_iter=4); eng2.set_mode(mode)
     eng2.step(40); eng2.sync(); cpu2.step(40)
-    assert len(cpu2.contacts()[0]) > 0 and rel_position_error(eng2.get_attr(_capi.ATTR_X), cpu2.get("x")) <= TOL
+    assert len(cpu2.oracle_contacts()[0]) > 0 and rel_position_error(eng2.get_attr(_capi.ATTR_X), cpu2.get("x")) <= TOL
     eng.close(); eng2.close()
 
 
 def test_tet_model_contacts_with_substeps(cpu_libs):
     """A tet model as the particle side (TetModelCollisionObjectType + rigid body: collisionDetectionRBSolid as well), two substeps per
     step: the contacts are detected and solved once per step, after the substeps (TimeStepController.cpp:189-196)."""
-    if not have_ref("f64"):
-        pytest.skip("prebuilt oracle/_ref/libpbdref_f64.so not present on this box")
-    from positionbaseddynamics_b200 import _capi
-    cpu = cpu_libs.CpuPbd("ref", "f64")
-    scenes.bar_on_colliders(cpu)
+    cpu = cpu_libs.CpuPbd("oracle", "f64")
+    colliders = scenes.on_recorded_colliders(cpu, "bar")
     cpu.init_groups()
-    eng = _engine_from(cpu)
+    eng = _engine_from(cpu, colliders)
     eng.set_params(dt=0.005, sub_steps=2, max_iter=3)
     n = cpu.num_particles()
     xo = np.zeros((n, 3), np.float32); vo = np.zeros((n, 3), np.float32)
@@ -142,13 +138,11 @@ def test_tet_model_contacts_with_substeps(cpu_libs):
 def test_contacts_matter_and_colliders_are_validated(cpu_libs):
     """Negative control: the same engine without the colliders leaves the tolerance by orders of magnitude; a collider on a dynamic body
     is refused."""
-    if not have_ref("f64"):
-        pytest.skip("prebuilt oracle/_ref/libpbdref_f64.so not present on this box")
     from positionbaseddynamics_b200 import _capi
-    cpu = cpu_libs.CpuPbd("ref", "f64")
-    scenes.cloth_on_colliders(cpu, 24, shapes=("box", "sphere", "torus"))
+    cpu = cpu_libs.CpuPbd("oracle", "f64")
+    scenes.on_recorded_colliders(cpu, "cloth_box_sphere_torus")
     cpu.init_groups()
-    eng = _engine_from(cpu, with_colliders=False)
+    eng = _engine_from(cpu)
     eng.set_params(dt=0.005, sub_steps=1, max_iter=4)
     eng.step(120); eng.sync(); cpu.step(120)
     assert rel_position_error(eng.get_attr(_capi.ATTR_X), cpu.get("x")) > 100 * TOL
@@ -164,13 +158,13 @@ def test_contacts_matter_and_colliders_are_validated(cpu_libs):
 def test_adapter_runs_the_contact_path(precision, cpu_libs):
     """The reference-side adapter with the reference's own DistanceFieldCollisionDetection attached (TimeStep::setCollisionDetection,
     as Demos/DistanceFieldDemos/ClothCollisionDemo.cpp:162-181): GpuTimeStepController reads the collision objects, the engine detects
-    and solves the contacts; twin on the reference's TimeStepController in fp64."""
+    and solves the contacts; twin on the fp64 checker."""
     from oracle import pyoracle
-    if not (pyoracle.available("refgpu", precision) and have_ref("f64")):
+    if not pyoracle.available("refgpu", precision):
         pytest.skip("prebuilt oracle/_ref/libpbdref_gpu_%s.so not present on this box" % precision)
-    gpu = cpu_libs.CpuPbd("refgpu", precision); cpu = cpu_libs.CpuPbd("ref", "f64")
-    for m in (gpu, cpu):
-        scenes.cloth_on_colliders(m, 24, shapes=ALL_SHAPES)
+    gpu = cpu_libs.CpuPbd("refgpu", precision); cpu = cpu_libs.CpuPbd("oracle", "f64")
+    scenes.cloth_on_colliders(gpu, 24, shapes=ALL_SHAPES)
+    scenes.on_recorded_colliders(cpu, "cloth_all_shapes")
     gpu.use_gpu_timestep(0, 0)
     gpu.set_contact_params(stiffness=100.0, max_iter_v=5)  # the parameter lives in the time step: set it on the installed one
     def step_gpu(x, v):
@@ -191,12 +185,10 @@ def test_adapter_runs_the_contact_path(precision, cpu_libs):
 def test_host_mirror_contact_path(cpu_libs):
     """The same scene through the host mirror of the reference's interface (C++ SimulationModel / TimeStepController /
     DistanceFieldCollisionDetection of csrc/host/pbd_model.h, driven through include/pbd_b200_model.h): addCollisionBox / Sphere / Torus on static
-    bodies, addCollisionObjectWithoutGeometry for the cloth, TimeStep::setCollisionDetection -- in lockstep with the reference."""
-    if not have_ref("f64"):
-        pytest.skip("prebuilt oracle/_ref/libpbdref_f64.so not present on this box")
+    bodies, addCollisionObjectWithoutGeometry for the cloth, TimeStep::setCollisionDetection -- in lockstep with the fp64 checker."""
     from positionbaseddynamics_b200 import _capi, model as hm_mod
-    cpu = cpu_libs.CpuPbd("ref", "f64")
-    bodies = scenes.cloth_on_colliders(cpu, 24, shapes=("box", "sphere", "torus"))
+    cpu = cpu_libs.CpuPbd("oracle", "f64")
+    scenes.on_recorded_colliders(cpu, "cloth_box_sphere_torus")
     hm = hm_mod.HostModel()
     hm.add_regular_triangle_model(24, 24, t=(-2.5, 2.2, -2.5), R=scenes.RX90, scale=(5.0, 5.0))
     hm.add_cloth_constraints(0, 4, dist_k=1.0e5)

@@ -8,6 +8,7 @@ against fp64 only: the fp32 reference is dominated by cancellation noise there (
 import numpy as np
 import pytest
 
+import reference_golden
 import scenes
 from parity_util import perturb, rel_position_error, rel_displacement_error
 from conftest import have_ref
@@ -76,10 +77,29 @@ def test_scene_vs_oracle_f64(name, cpu_libs):
 
 
 @pytest.mark.parametrize("name", sorted(SCENES))
-def test_scene_vs_reference_f64(name, cpu_libs):
-    if not have_ref("f64"):
-        pytest.skip("prebuilt oracle/_ref/libpbdref_f64.so not present on this box")
-    _run(name, 0, cpu_libs, "ref")
+def test_scene_vs_reference_f64(name):
+    """The same gates as _run, with the reference's recorded fp64 run of the scene (tests/golden/reference_runs.npz) as the checker:
+    structure bit for bit, positions on the recorded sample of particles, relative to the scales of the whole run."""
+    from positionbaseddynamics_b200.model import HostModel
+    build, amp, steps = SCENES[name]
+    key = "gpu_parity/%s/" % name
+    gpu = HostModel()
+    build(gpu)
+    tg, bg, _, _ = gpu.constraints()
+    reference_golden.assert_structure(key, tg, bg, *gpu.groups())
+    perturb([gpu], amp)
+    gpu.time_step().set_mode(0)
+    gpu.step(steps)
+    xg = gpu.get("x")
+    assert np.isfinite(xg).all()
+    x_ref, x_got, x_scale = reference_golden.sampled(key, "x", xg)
+    d = np.abs(x_got.astype(np.float64) - x_ref).max()
+    e_pos, e_disp = d / x_scale, d / reference_golden.get(key + "disp_scale")
+    print("%s vs recorded reference: rel pos %.2e, rel disp %.2e" % (name, e_pos, e_disp))
+    assert e_pos <= (5e-4 if name == "bar_femtet_xpbd" else TOL), (name, e_pos)
+    if name != "bar_femtet_xpbd":
+        assert e_disp <= TOL_DISP, (name, e_disp)
+    gpu.close()
 
 
 @pytest.mark.parametrize("name", ["cloth_isobending_xpbd", "bar_fem_plus_volume", "cfg1_50x50", "mixed_cloth_solid"])

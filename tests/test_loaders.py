@@ -1,9 +1,8 @@
 """Mesh import with the reference's names (SURVEY.md section 8 row f-4, import part): Utilities::TetGenLoader / OBJLoader semantics
-(Utils/TetGenLoader.cpp, Utils/OBJLoader.h) on small committed files, and -- where the reference tree is present -- on its own
-data/models/armadillo_4k.{node,ele}, whose tet model is then built by the host mirror and by the reference from the same arrays."""
+(Utils/TetGenLoader.cpp, Utils/OBJLoader.h) on small committed files, and on the reference's own data/models/armadillo_4k mesh,
+whose tet model is then built by the host mirror and held against the reference's."""
 import os
 import numpy as np
-import pytest
 
 import positionbaseddynamics_b200.pypbd as pbd
 
@@ -34,21 +33,31 @@ def test_obj_loader():
     assert tm.getParticleMesh().numFaces() == 2 and tm.getParticleMesh().numEdges() == 5
 
 
-def test_armadillo_tet_model_like_the_reference(cpu_libs):
-    node, ele = "/root/reference/data/models/armadillo_4k.node", "/root/reference/data/models/armadillo_4k.ele"
-    if not (os.path.exists(node) and os.path.exists(ele)):
-        pytest.skip("reference data files not present on this box")
+def test_armadillo_tet_model_like_the_reference(tmp_path, cpu_libs):
+    """The reference's armadillo_4k mesh (as its TetGen loader reads it, tests/golden/reference_runs.npz) written back in TetGen format,
+    loaded, and built into a tet model by the host mirror and the C restatement: the same colouring and edges as the reference's model."""
+    import reference_golden as rg
+    x_ref, t_ref = rg.get("armadillo/x"), rg.get("armadillo/tets")
+    node, ele = str(tmp_path / "armadillo_4k.node"), str(tmp_path / "armadillo_4k.ele")
+    with open(node, "w") as f:
+        f.write("%d  3  0  0\n" % len(x_ref) + "".join("%4d    %r  %r  %r\n" % ((i,) + tuple(map(float, p))) for i, p in enumerate(x_ref)))
+    with open(ele, "w") as f:
+        f.write("%d  4  0\n" % len(t_ref) + "".join("%5d     %d  %d  %d  %d\n" % ((i,) + tuple(map(int, q))) for i, q in enumerate(t_ref)))
     x, t = pbd.TetGenLoader.loadTetgenModel(node, ele)
     assert x.shape == (1180, 3) and len(t) == 4 * 3717
+    assert (x == x_ref).all() and (t.reshape(-1, 4) == t_ref).all()
     from positionbaseddynamics_b200.model import HostModel
-    from conftest import have_ref
-    hm = HostModel(); other = cpu_libs.CpuPbd("ref" if have_ref("f64") else "oracle", "f64")
+    hm = HostModel(); other = cpu_libs.CpuPbd("oracle", "f64")
     for m in (hm, other):
         m.add_tet_model(x, t.reshape(-1, 4))
         m.add_solid_constraints(0, 2, k=1.0e6, nu=0.3)
     hm.init_groups(); other.init_groups()
     assert hm.num_constraints() == other.num_constraints() == 3717
-    off_a, ids_a = hm.groups(); off_b, ids_b = other.groups()
-    assert (off_a == off_b).all() and (ids_a == ids_b).all()          # same colouring of the imported mesh
+    types, bodies, _, _ = hm.constraints()
+    rg.assert_structure("armadillo/", types, bodies, *hm.groups())     # the reference's colouring of the imported mesh
+    off_b, ids_b = other.groups()
+    off_a, ids_a = hm.groups()
+    assert (off_a == off_b).all() and (ids_a == ids_b).all()
+    assert (rg.digest(hm.tet_edges(0), np.uint32) == rg.get("armadillo/tet_edges")).all()
     assert (hm.tet_edges(0) == other.tet_edges(0)).all()
     hm.close()

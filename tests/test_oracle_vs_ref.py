@@ -1,8 +1,9 @@
-"""Oracle pinned against the reference itself (oracle/_ref), where the prebuilt library is present (the build container
-and, because oracle/_ref travels with the snapshot, the GPU box).  Larger than the golden fixtures."""
+"""Oracle pinned against the reference itself: against its recorded runs (tests/golden/reference_runs.npz) everywhere, and against
+a reference build (oracle/_ref) where one was made.  Larger than the golden fixtures."""
 import numpy as np
 import pytest
 
+import reference_golden
 import scenes
 from conftest import have_ref
 from parity_util import perturb
@@ -20,23 +21,25 @@ CASES = {
 }
 
 
-@needs_ref
+def steps_of(name):
+    return 1 if name.endswith("1step") else 3  # XPBD-FEM amplifies rounding differences chaotically after a step
+
+
 @pytest.mark.parametrize("name", sorted(CASES))
 def test_structure_and_trajectory(name, cpu_libs):
+    """The reference's side is the recorded run of tests/golden/reference_runs.npz (same builder, perturbation and steps)."""
     for prec, tol in (("f64", 1e-9), ("f32", 5e-5)):
-        o = cpu_libs.CpuPbd("oracle", prec); r = cpu_libs.CpuPbd("ref", prec)
-        for m in (o, r):
-            CASES[name](m)
-        to, bo, po, _ = o.constraints(); tr, br, pr, _ = r.constraints()
-        assert (to == tr).all() and (bo == br).all()
-        go, gr = o.groups(), r.groups()
-        assert (go[0] == gr[0]).all() and (go[1] == gr[1]).all()
-        assert np.abs(po - pr).max() <= tol * max(np.abs(pr).max(), 1.0)
-        perturb([o, r], 0.01)
-        steps = 1 if name.endswith("1step") else 3  # XPBD-FEM amplifies rounding differences chaotically after a step
-        o.step(steps); r.step(steps)
-        xo, xr = o.get("x"), r.get("x")
-        err = np.abs(xo - xr).max() / np.abs(xr).max()
+        key = "oracle_vs_ref/%s/%s/" % (name, prec)
+        o = cpu_libs.CpuPbd("oracle", prec)
+        CASES[name](o)
+        to, bo, po, _ = o.constraints()
+        reference_golden.assert_structure(key, to, bo, *o.groups())
+        p_ref, p_got, p_scale = reference_golden.sampled(key, "params", po, reference_golden.PARAM_ROWS)
+        assert np.abs(p_got - p_ref).max() <= tol * p_scale
+        perturb([o], 0.01)
+        o.step(steps_of(name))
+        x_ref, x_got, x_scale = reference_golden.sampled(key, "x", o.get("x"))
+        err = np.abs(x_got - x_ref).max() / x_scale
         limit = tol
         if prec == "f32" and name in ("cfg1", "cloth_xpbd_64"):
             limit = 3e-3  # isometric bending in fp32: both sides are inside the reference's own cancellation noise
@@ -81,44 +84,56 @@ def test_reference_side_adapter_is_built_and_fails_loudly_without_a_gpu():
             assert np.abs(m.get("x") - x0).max() > 0
 
 
+CONTACT_STEPS = 110
+CHECKPOINTS = (40, 60, 80, 100, 110)  # fp64: velocities compared along the free run (the first contacts appear around step 35)
+LOCKSTEP_STEPS = (60, 90)             # fp32: single steps from the reference's state
+
+
 @pytest.mark.parametrize("precision", ["f64", "f32"])
 def test_contact_path_restatement_is_pinned_to_the_reference(precision, cpu_libs):
     """The C restatement of the contact path (oracle/pbd_oracle.c: distance functions, collisionTest, contact initialisation, velocity-level
-    solve) against the reference's DistanceFieldCollisionDetection + ParticleRigidBodyContactConstraint in the same precision: in lockstep
-    (the oracle takes the reference's state before every step) over 110 steps of a cloth falling onto all six analytic shapes -- the same
-    contact list, and velocities that agree to rounding (the two sides evaluate the same formulas in the same precision)."""
-    if not have_ref(precision):
-        pytest.skip("prebuilt oracle/_ref/libpbdref_%s.so not present" % precision)
-    ref = cpu_libs.CpuPbd("ref", precision); orc = cpu_libs.CpuPbd("oracle", precision)
+    solve) against the reference's DistanceFieldCollisionDetection + ParticleRigidBodyContactConstraint in the same precision, as recorded
+    in tests/golden/reference_runs.npz: 110 steps of a cloth falling onto all six analytic shapes -- the same contact list after every
+    step, and velocities that agree to rounding (the two sides evaluate the same formulas in the same precision).  In fp64 the velocities
+    are compared along the free run; in fp32, whose rounding differences grow over a free run, after single steps taken from the
+    reference's state."""
     # Real = float: the reference takes the torus' ring distance from a float norm (Vector2r(x, z).norm(), DistanceFieldCollisionDetection.cpp:635);
     # the central differences of approximateNormal (eps = 1e-6) then differentiate rounding noise and the normal is off by percent in a
     # rounding-dependent direction -- nothing to pin there, so the float run leaves the torus out (the double run has all six shapes)
-    shapes = ("box", "sphere", "torus", "cylinder", "hollow_sphere", "hollow_box") if precision == "f64" else ("box", "sphere", "cylinder", "hollow_sphere", "hollow_box")
-    scenes.cloth_on_colliders(ref, 24, shapes=shapes)
-    orc.add_regular_triangle_model(24, 24, t=(-2.5, 2.2, -2.5), R=scenes.RX90, scale=(5.0, 5.0))
-    orc.add_cloth_constraints(0, 4, dist_k=1.0e5)
-    orc.add_bending_constraints(0, 3, 100.0)
-    orc.set_params(dt=0.005, sub_steps=1, max_iter=4)
-    for row in ref.rigid_bodies():
-        orc.add_rigid_body(0.0, row[:3], (1.0, 1.0, 1.0), row[3:7])
-    models, rigid = ref.collision_objects()
-    orc.set_colliders(models, rigid)
-    orc.set_oracle_contact_params(tolerance=0.05, stiffness=100.0, max_iter_v=5)
-    events = 0; worst_dv = 0.0; worst_x = 0.0; grazing = 0
-    tol_v = 1e-9 if precision == "f64" else 5e-3  # float: the penalty impulse (stiffness 100 x depth) amplifies the rounding of the positions; a flipped contact would be 0.1 - 2 m/s
-    for step in range(110):
-        orc.set("x", ref.get("x")); orc.set("v", ref.get("v"))
-        ref.step(1); orc.step(1)
-        p, b, info, rr, pt = ref.contacts()
-        po, bo, io = orc.oracle_contacts()
-        a, c = set(zip(p.tolist(), b.tolist())), set(zip(po.tolist(), bo.tolist()))
+    orc = cpu_libs.CpuPbd("oracle", precision)
+    scenes.on_recorded_colliders(orc, "cloth_all_shapes" if precision == "f64" else "cloth_no_torus_f32")
+    key = "contact_run/%s/" % precision
+    counts = reference_golden.get(key + "counts"); pairs = [tuple(q) for q in reference_golden.get(key + "pairs").tolist()]
+    starts = np.concatenate([[0], np.cumsum(counts, dtype=np.int64)])
+    events = 0; worst_dv = 0.0; grazing = 0
+
+    def compare_contacts(step):
+        a = set(pairs[starts[step - 1]:starts[step]])  # the reference's contacts of this step
+        po, bo, _ = orc.oracle_contacts()
+        c = set(zip(po.tolist(), bo.tolist()))
         if a != c:  # only a contact whose signed distance is at the rounding level may be on one side only (never in fp64)
             assert precision == "f32" and len(a ^ c) <= 2, "step %d: contact lists differ: %s" % (step, sorted(a ^ c))
-            grazing += len(a ^ c)
-        events += len(p)
-        worst_x = max(worst_x, float(np.abs(orc.get("x") - ref.get("x")).max()))
-        dv = np.abs(orc.get("v") - ref.get("v")).max(axis=1)
-        dv[[q for q, _ in a ^ c]] = 0.0
-        worst_dv = max(worst_dv, float(dv.max()))
-    print("contact restatement, %s: %d contact events, %d grazing, worst |dx| %.2e, worst |dv| %.2e" % (precision, events, grazing, worst_x, worst_dv))
+        return a, a ^ c
+
+    def velocity_error(step, one_sided):
+        v_ref, v_got, _ = reference_golden.sampled(key, "v%d" % step, orc.get("v"))
+        dv = np.abs(v_got - v_ref).max(axis=1)
+        dv[np.isin(reference_golden.sample_rows(orc.num_particles()), [q for q, _ in one_sided])] = 0.0
+        return float(dv.max())
+
+    tol_v = 1e-9 if precision == "f64" else 5e-3  # float: the penalty impulse (stiffness 100 x depth) amplifies the rounding of the positions; a flipped contact would be 0.1 - 2 m/s
+    for step in range(1, CONTACT_STEPS + 1):
+        orc.step(1)
+        a, one_sided = compare_contacts(step)
+        grazing += len(one_sided); events += len(a)
+        if precision == "f64" and step in CHECKPOINTS:
+            worst_dv = max(worst_dv, velocity_error(step, one_sided))
+    if precision == "f32":
+        for step in LOCKSTEP_STEPS:
+            orc.set("x", reference_golden.get(key + "x_before%d" % step)); orc.set("v", reference_golden.get(key + "v_before%d" % step))
+            orc.step(1)
+            _, one_sided = compare_contacts(step)
+            grazing += len(one_sided)
+            worst_dv = max(worst_dv, velocity_error(step, one_sided))
+    print("contact restatement, %s: %d contact events, %d grazing, worst |dv| %.2e" % (precision, events, grazing, worst_dv))
     assert events > 2000 and grazing <= 4 and worst_dv <= tol_v

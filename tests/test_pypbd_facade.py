@@ -136,22 +136,19 @@ def test_mass_properties_and_rigid_body_facade():
         model.addRigidBody(1.0, CUBE_V, CUBE_F, generateCollisionObject=True)
 
 
-@pytest.mark.gpu
-def test_coupling_example_against_the_reference(cpu_libs):
-    """examples/rigid_body_cloth_coupling.py (pyPBD-style construction incl. mesh-derived mass properties) stepped on the GPU, against
-    the unmodified reference given the same bodies (mass, position, principal inertia, rotation)."""
+def coupling_example_model():
+    """(example module, model) of examples/rigid_body_cloth_coupling.py, built through the facade."""
     import importlib.util, os
     import positionbaseddynamics_b200.pypbd as pbd
-    from conftest import have_ref
-    if not have_ref("f64"):
-        pytest.skip("prebuilt oracle/_ref/libpbdref_f64.so not present on this box")
     pbd.Simulation._current = None
     root = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "examples")
     spec = importlib.util.spec_from_file_location("rigid_body_cloth_coupling", os.path.join(root, "rigid_body_cloth_coupling.py"))
     ex = importlib.util.module_from_spec(spec); spec.loader.exec_module(ex)
-    model = ex.buildModel()
-    host = model._host
-    ref = cpu_libs.CpuPbd("ref", "f64")
+    return ex, ex.buildModel()
+
+
+def coupling_example_on_cpu(ref, ex, host):
+    """The example's scene on a CPU checker, given the same bodies (mass, position, principal inertia, rotation) as the facade's."""
     ref.add_regular_triangle_model(ex.nCols, ex.nRows, [-5, 4, -5], ex.rotation_x(np.pi * 0.5), [ex.clothWidth, ex.clothHeight])
     ref.add_cloth_constraints(0, 2, 1.0, 1.0, 1.0, 1.0, 0.3, 0.3)
     ref.add_bending_constraints(0, 2, 0.01)
@@ -169,16 +166,26 @@ def test_coupling_example_against_the_reference(cpu_libs):
     for body, particle in ((2, 0), (5, ex.nCols - 1), (8, ex.nRows * ex.nCols - 1), (11, (ex.nRows - 1) * ex.nCols)):
         ref.add_rb_particle_ball_joint(body, particle)
     ref.set_params(dt=0.005, sub_steps=3, max_iter=1)
-    assert ref.num_constraints() == model.numConstraints()
+
+
+@pytest.mark.gpu
+def test_coupling_example_against_the_reference():
+    """examples/rigid_body_cloth_coupling.py (pyPBD-style construction incl. mesh-derived mass properties) stepped on the GPU, against
+    the unmodified reference given the same bodies (coupling_example_on_cpu): its recorded run, tests/golden/reference_runs.npz."""
+    import positionbaseddynamics_b200.pypbd as pbd
+    import reference_golden as rg
+    _, model = coupling_example_model()
+    host = model._host
+    assert rg.get("coupling_example/num_constraints") == model.numConstraints()
     sim = pbd.Simulation.getCurrent()
     for _ in range(6):
         sim.getTimeStep().step(model)
-    ref.step(6)
-    xg = model.getParticles().getVertices(); xc = ref.get("x")
-    err = np.abs(xg - xc).max() / np.abs(xc).max()
+    xg = model.getParticles().getVertices()
+    x_ref, x_got, x_scale = rg.sampled("coupling_example/", "x", xg)
+    err = np.abs(x_got - x_ref).max() / x_scale
     print("coupling example vs reference: rel pos %.2e" % err)
     assert err <= 1e-4
-    assert np.abs(host.rigid_bodies()[:, :3] - ref.rigid_bodies()[:, :3]).max() <= 1e-4
+    assert np.abs(host.rigid_bodies()[:, :3] - rg.get("coupling_example/rb_x")).max() <= 1e-4
 
 
 def _quat_to_matrix(q):
@@ -188,20 +195,21 @@ def _quat_to_matrix(q):
                      [2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)]])
 
 
-def test_facade_rigid_body_matches_the_reference_init(cpu_libs):
+RB_R0 = np.array([[np.cos(0.3), -np.sin(0.3), 0], [np.sin(0.3), np.cos(0.3), 0], [0, 0, 1.0]])
+RB_VERTS = CUBE_V + [0.1, 0.2, 0.3]          # off-centre: the body frame has to move to the centre of mass
+RB_SCALES = ([0.4, 2.0, 0.6], [1.0, 1.0, 3.0])
+
+
+def test_facade_rigid_body_matches_the_reference_init():
     """addRigidBody(density, vertices, mesh, translation, rotation, scale) against the unmodified reference's
-    RigidBody::initBody(density, ...) (Utils/VolumeIntegration.cpp + principal-axes transform): mass, principal moments, position and
-    the world-space inertia tensor (the principal frame itself is only defined up to signs / degenerate subspaces)."""
-    from conftest import have_ref
+    RigidBody::initBody(density, ...) (Utils/VolumeIntegration.cpp + principal-axes transform), as recorded in
+    tests/golden/reference_runs.npz: mass, principal moments, position and the world-space inertia tensor (the principal frame
+    itself is only defined up to signs / degenerate subspaces)."""
     import positionbaseddynamics_b200.pypbd as pbd
-    if not have_ref("f64"):
-        pytest.skip("oracle/_ref not built")
-    a = 0.3
-    R0 = np.array([[np.cos(a), -np.sin(a), 0], [np.sin(a), np.cos(a), 0], [0, 0, 1.0]])
-    verts = CUBE_V + [0.1, 0.2, 0.3]          # off-centre: the body frame has to move to the centre of mass
-    for scale in ([0.4, 2.0, 0.6], [1.0, 1.0, 3.0]):
-        ref = cpu_libs.CpuPbd("ref", "f64")
-        _, props = ref.add_rigid_body_mesh(2.0, verts, CUBE_F, x=(1.0, 2.0, 3.0), R=R0, scale=scale)
+    import reference_golden as rg
+    R0, verts = RB_R0, RB_VERTS
+    for k, scale in enumerate(RB_SCALES):
+        props = rg.get("facade_rigid_body/%d/props" % k)
         pbd.Simulation._current = None
         sim = pbd.Simulation.getCurrent(); sim.initDefault(); model = sim.getModel()
         rb = model.addRigidBody(2.0, verts, CUBE_F, translation=[1.0, 2.0, 3.0], rotation=R0, scale=scale)
