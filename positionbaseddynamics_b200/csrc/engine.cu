@@ -810,9 +810,11 @@ static int choose_resident_shape(pbd_engine *e) {
     // the block sizes the instantiations compile for without spilling (cloth 96 registers, light 128, everything 236)
     e->resThreads = (e->resMask == kMaskClothXPBD) ? 640u : ((e->resMask == kMaskAll) ? 256u : 512u);
     if (const char *g = getenv("PBD_B200_RTHREADS")) { const int k = atoi(g); if (k == 256 || k == 512 || k == 640 || k == 768) e->resThreads = (unsigned)k; }
-    if (e->resMask == kMaskAll && e->resThreads > 512u) e->resThreads = 512u;
+    // clamp to a block size the mask is instantiated for (with_resident_kernel): the kernel's THREADS must equal the launch's block size.
+    // cloth-XPBD 512 / 640 / 768, cloth and light 512, FEM / solid / everything 256 / 512
     if (e->resMask == kMaskLight || e->resMask == kMaskCloth) e->resThreads = 512u;
-    if (e->resMask == kMaskClothXPBD && e->resThreads == 256u) e->resThreads = 512u;
+    else if (e->resMask == kMaskClothXPBD) { if (e->resThreads < 512u) e->resThreads = 512u; }
+    else if (e->resThreads > 512u) e->resThreads = 512u;
     const unsigned nGroups = (unsigned)std::max<size_t>(e->groupOff.size(), 2) - 1;
     const unsigned perPhase = e->numConstraints / std::max(1u, nGroups);
     // particles a tile can hold: what is left of the CTA's shared memory after the phase tables (bound: one bucket per colour and type)

@@ -11,7 +11,9 @@ from conftest import have_ref
 pytestmark = pytest.mark.gpu
 
 
-def _gpu(build, mode=0):
+def _gpu(build, mode=4):
+    """The scene on a GPU time step; the default is PBD_MODE_AUTO, what a user and bench.py run (the resident kernel for cfg2, cfg3
+    and cfg5); the bitwise tests below hold the other modes to it."""
     from positionbaseddynamics_b200.model import HostModel
     m = HostModel(); build(m); m.time_step().set_mode(mode)
     return m

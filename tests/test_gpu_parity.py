@@ -102,15 +102,6 @@ def test_scene_vs_reference_f64(name):
     gpu.close()
 
 
-@pytest.mark.parametrize("name", ["cloth_isobending_xpbd", "bar_fem_plus_volume", "cfg1_50x50", "mixed_cloth_solid"])
-def test_modes_agree_bitwise(name, cpu_libs):
-    """Plain launches, the replayed CUDA graph and the resident cluster kernel (positions in distributed shared memory, tile-major
-    particle order) execute the same projections in the same dependency order, so their results must be bit-identical."""
-    xs = [_run(name, mode, cpu_libs, "oracle") for mode in (2, 0, 1)]
-    assert (xs[0] == xs[1]).all()
-    assert (xs[0] == xs[2]).all()
-
-
 def test_mode_switch_keeps_state_bitwise():
     """Switching to the resident mode permutes every particle array on the device (tile-major order) and back; the simulation
     state must survive both moves bit for bit and the uploads/downloads in between must address the right particles."""
@@ -156,6 +147,18 @@ def test_reference_side_adapter(name, precision, cpu_libs):
     installed with Simulation::setTimeStep.  The REFERENCE builds the scene, initialises the constraints and colours them; the
     adapter flattens the model through its public members and steps it with libpbd_b200.so.  A twin scene stepped by the
     reference's own TimeStepController (fp64) is the yardstick."""
+    _reference_side_adapter(name, precision, 0, cpu_libs)
+
+
+@pytest.mark.parametrize("precision", ["f32", "f64"])
+@pytest.mark.parametrize("name", ADAPTER_SCENES)
+def test_reference_side_adapter_auto_mode(name, precision, cpu_libs):
+    """test_reference_side_adapter with the adapter in PBD_MODE_AUTO, the default of a user: the resident kernel for the cloth and
+    FEM scenes, the graph mode for the others."""
+    _reference_side_adapter(name, precision, 4, cpu_libs)
+
+
+def _reference_side_adapter(name, precision, mode, cpu_libs):
     from oracle import pyoracle
     if not (pyoracle.available("refgpu", precision) and have_ref("f64")):
         pytest.skip("prebuilt oracle/_ref/libpbdref_gpu_%s.so not present on this box" % precision)
@@ -165,14 +168,14 @@ def test_reference_side_adapter(name, precision, cpu_libs):
         build, amp, steps = SCENES[name]
     gpu = cpu_libs.CpuPbd("refgpu", precision); cpu = cpu_libs.CpuPbd("ref", "f64")
     build(gpu); build(cpu)
-    gpu.use_gpu_timestep(0, 0)
+    gpu.use_gpu_timestep(0, mode)
     x_start = perturb([gpu, cpu], amp) if amp else cpu.get("x")
     gpu.step(steps); cpu.step(steps)
     assert gpu.gpu_error() == ""
     xg, xc = gpu.get("x"), cpu.get("x")
     assert np.isfinite(xg).all()
     e_pos = rel_position_error(xg, xc)
-    print("adapter %s Real=%s: rel pos %.2e" % (name, precision, e_pos))
+    print("adapter %s Real=%s mode %d: rel pos %.2e" % (name, precision, mode, e_pos))
     assert e_pos <= TOL, (name, e_pos)
     assert abs(gpu.time() - cpu.time()) < 1e-6       # TimeManager advanced like TimeStepController.cpp:239
     if name == "cfg4_small_with_rig":
@@ -234,10 +237,37 @@ def test_device_colouring_more_than_128_colours():
     eng.close()
 
 
-def test_known_answers_against_reference_golden():
-    """Per-function known answers: the golden inputs/outputs recorded from the reference's stateless solve_* functions
-    (tests/golden/kat_f64.npz) replayed through the CUDA kernels.  Every case becomes one constraint on four private
-    particles (one colour, no coupling), gravity off, 1 substep x 1 iteration, so x_after - x_before is the correction."""
+def _kat_engine(x, w, cases, dt, mode, clusters=None):
+    """One engine holding `cases` = [(type, params row)], case j on particles 4j..4j+3: one step of 1 substep x 1 iteration without
+    gravity.  Returns the corrections [len(cases), 4, 3] and the multipliers by case (NaN for non-XPBD types)."""
+    import os
+    from positionbaseddynamics_b200 import _capi
+    if clusters:
+        os.environ["PBD_B200_CLUSTERS"] = clusters
+    try:
+        eng = _capi.Engine(0)
+        try:
+            mass = np.where(w != 0, 1.0 / np.where(w != 0, w, 1.0), 0.0).astype(np.float32)
+            eng.set_particles(x, mass)
+            for j, (t, p) in enumerate(cases):
+                eng.add_constraints(t, np.arange(4 * j, 4 * j + _capi.num_bodies(t)), p[:_capi.num_params(t)])
+            eng.color_first_fit()
+            eng.set_params(dt=float(dt), sub_steps=1, max_iter=1, gravity=(0, 0, 0))
+            eng.set_mode(mode)
+            eng.step(1); eng.sync()
+            got = (eng.get_attr(_capi.ATTR_X).astype(np.float64) - x.astype(np.float64)).reshape(-1, 4, 3)
+            lam = np.full(len(cases), np.nan)
+            for t in (_capi.DISTANCE_XPBD, _capi.ISOBENDING_XPBD, _capi.VOLUME_XPBD, _capi.FEMTET_XPBD):
+                if any(c[0] == t for c in cases):
+                    vals, ids = eng.lambdas(t); lam[ids] = vals
+        finally:
+            eng.close()
+    finally:
+        os.environ.pop("PBD_B200_CLUSTERS", None)
+    return got, lam
+
+
+def _known_answers(mode, clusters=None):
     import os
     from positionbaseddynamics_b200 import _capi
     d = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "kat_f64.npz"))
@@ -249,22 +279,12 @@ def test_known_answers_against_reference_golden():
         if T[i] in (_capi.FEMTET, _capi.FEMTET_XPBD):
             x = X[i]; vol = np.dot(np.cross(x[1] - x[0], x[2] - x[0]), x[3] - x[0]) / 6.0
             ok[i] &= (bool(d["solve_hinv"][i]) == bool(vol / P[i][0] < 0.2))
-    worst = {}
+    worst = {}; worst_lam = 0.0
     for dt in np.unique(DT):
         sel = np.nonzero(ok & (DT == dt))[0]
-        eng = _capi.Engine(0)
         x = X[sel].reshape(-1, 3).astype(np.float32)
         w = W[sel].reshape(-1)
-        mass = np.where(w != 0, 1.0 / np.where(w != 0, w, 1.0), 0.0).astype(np.float32)
-        eng.set_particles(x, mass)
-        for j, i in enumerate(sel):
-            t = int(T[i]); nb = _capi.num_bodies(t)
-            eng.add_constraints(t, np.arange(4 * j, 4 * j + nb), P[i][:_capi.num_params(t)])
-        eng.color_first_fit()
-        eng.set_params(dt=float(dt), sub_steps=1, max_iter=1, gravity=(0, 0, 0))
-        eng.set_mode(_capi.MODE_LAUNCH)
-        eng.step(1); eng.sync()
-        got = (eng.get_attr(_capi.ATTR_X).astype(np.float64) - x.astype(np.float64)).reshape(-1, 4, 3)
+        got, lam = _kat_engine(x, w, [(int(T[i]), P[i]) for i in sel], dt, mode, clusters)
         for j, i in enumerate(sel):
             ref = d["solve_corr"][i].copy()
             if not d["solve_res"][i]:
@@ -275,9 +295,75 @@ def test_known_answers_against_reference_golden():
             worst[int(T[i])] = max(worst.get(int(T[i]), 0.0), err)
             # fp32 kernels vs fp64 reference answers on O(1) stencils a few units from the origin
             assert err <= 5e-4, (int(T[i]), int(i), err, got[j], ref)
-        eng.close()
-    print("GPU known answers, worst relative error per type:", {_capi.TYPE_NAMES[k]: "%.1e" % v for k, v in sorted(worst.items())})
+            if not np.isnan(lam[j]):  # XPBD: the multiplier after the solve
+                e_lam = abs(lam[j] - d["solve_lam1"][i]) / max(abs(d["solve_lam1"][i]), 1e-3)
+                worst_lam = max(worst_lam, e_lam)
+                assert e_lam <= 5e-4, (int(T[i]), int(i), e_lam, lam[j], d["solve_lam1"][i])
+    print("GPU known answers (mode %d%s), worst relative error per type:" % (mode, ", clusters " + clusters if clusters else ""),
+          {_capi.TYPE_NAMES[k]: "%.1e" % v for k, v in sorted(worst.items())}, "multipliers %.1e" % worst_lam)
     assert len(worst) == 13
+
+
+def test_known_answers_against_reference_golden():
+    """Per-function known answers: the golden inputs/outputs recorded from the reference's stateless solve_* functions
+    (tests/golden/kat_f64.npz) replayed through the CUDA kernels.  Every case becomes one constraint on four private
+    particles (one colour, no coupling), gravity off, 1 substep x 1 iteration, so x_after - x_before is the correction."""
+    from positionbaseddynamics_b200 import _capi
+    _known_answers(_capi.MODE_LAUNCH)
+
+
+@pytest.mark.parametrize("mode", ["graph", "resident", "resident_4x1", "jacobi"])
+def test_known_answers_through_every_mode(mode):
+    """The known answers of test_known_answers_against_reference_golden through the other execution paths: the graph mode, the
+    resident kernel (its default shape, one cluster; and 4 independent CTAs, where stencils split between CTAs run as X items through
+    global memory) and the Jacobi mode, which equals Gauss-Seidel here because no two cases share a particle."""
+    from positionbaseddynamics_b200 import _capi
+    m, clusters = {"graph": (_capi.MODE_GRAPH, None), "resident": (_capi.MODE_RESIDENT, None),
+                   "resident_4x1": (_capi.MODE_RESIDENT, "4x1"), "jacobi": (_capi.MODE_JACOBI, None)}[mode]
+    _known_answers(m, clusters)
+
+
+def test_known_answers_full_q_bending(cpu_libs):
+    """IsometricBending with a Q that is not of the rank-one form (a user-modified Q): the full-Q projection (layout variant 1) of the
+    launch, graph and Jacobi modes against the fp64 checker's solver on the same parameter row; the resident mode refuses it."""
+    import os
+    from positionbaseddynamics_b200 import _capi
+    d = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "kat_f64.npz"))
+    T = d["solve_type"]
+    sel = np.nonzero(np.isin(T, (_capi.ISOBENDING, _capi.ISOBENDING_XPBD)) & (d["solve_lam0"] == 0.0))[0]
+    rng = np.random.RandomState(31)
+    rows = []
+    for i in sel:
+        p = d["solve_p"][i].copy()
+        Q = p[1:17].reshape(4, 4)
+        S = rng.uniform(-1.0, 1.0, (4, 4)); S = 0.5 * (S + S.T)
+        p[1:17] = (Q + 0.3 * np.abs(Q).max() * S).reshape(-1)
+        rows.append(p.astype(np.float32).astype(np.float64))  # what the engine sees, exactly
+    cpu = cpu_libs.CpuPbd("oracle", "f64")
+    worst = 0.0
+    for dt in np.unique(d["solve_dt"][sel]):
+        js = [j for j, i in enumerate(sel) if d["solve_dt"][i] == dt]
+        x = d["solve_x"][sel[js]].reshape(-1, 3).astype(np.float32)
+        w = d["solve_w"][sel[js]].reshape(-1)
+        cases = [(int(T[sel[j]]), rows[j]) for j in js]
+        ref = []
+        for k, j in enumerate(js):
+            res, corr, lam = cpu.kat_solve(cases[k][0], x[4 * k:4 * k + 4].astype(np.float64), w[4 * k:4 * k + 4], rows[j], dt=float(dt))
+            corr = corr if res else np.zeros((4, 3))
+            corr[w[4 * k:4 * k + 4] == 0] = 0.0
+            ref.append((corr, lam))
+        for mode in (_capi.MODE_LAUNCH, _capi.MODE_GRAPH, _capi.MODE_JACOBI):
+            got, lam = _kat_engine(x, w, cases, dt, mode)
+            for k in range(len(js)):
+                corr, lam_ref = ref[k]
+                err = np.abs(got[k] - corr).max() / max(np.abs(corr).max(), 1e-3)
+                worst = max(worst, err)
+                assert err <= 5e-4, (mode, cases[k][0], err, got[k], corr)
+                if cases[k][0] == _capi.ISOBENDING_XPBD:
+                    assert abs(lam[k] - lam_ref) <= 5e-4 * max(abs(lam_ref), 1e-3), (mode, lam[k], lam_ref)
+        with pytest.raises(_capi.PbdError):
+            _kat_engine(x, w, cases, dt, _capi.MODE_RESIDENT)
+    print("full-Q IsometricBending known answers: worst relative error %.1e" % worst)
 
 
 def test_engine_level_drop_in(cpu_libs):
